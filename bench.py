@@ -4,7 +4,7 @@
 Metric (BASELINE.json): Gauss-Newton/LM iterations per second on the 200-keyframe /
 20k-landmark synthetic double window (config C2), 10 iterations per step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one svs_ba_optimize(num_iters=10) over the whole window, starting from the same
 initial state (svs_ba_reset_state, device-to-device).  `value` counts iterations with the
@@ -15,6 +15,11 @@ replicas, no data-path collective), value = total iterations / max-over-ranks ti
 
 --impl reference times the CPU oracle (oracle/ba_oracle.c, the restatement of the reference's
 g2o path; the reference itself cannot be built here, see DESIGN.md) on the host cores.
+
+--dump-outputs DIR writes what the last timed step of rank 0 returned, after the timed region, as
+float64 arrays: DIR/poses.npy (P x 7, [q|t]), DIR/psi.npy (L x 3, inverse depth) and DIR/chi2_iter.npy
+(chi2 after every LM iteration).  The inputs are seeded, so two builds can be compared output for output;
+both arms write the same names.
 """
 from __future__ import annotations
 
@@ -105,6 +110,13 @@ def solve_kernel_bytes(st, pb):
     return 288 * 3 * st["nnzb_L"] + 144 * pb.P
 
 
+def dump_outputs(out_dir, poses, psi, chi2_iter):
+    """The arrays a caller of the timed step receives, as float64 .npy files (about 0.5 MB for C2)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("poses", poses), ("psi", psi), ("chi2_iter", chi2_iter)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def cpu_mt_sample(po, pb, seconds=4.0):
     """The oracle's multi-threaded timing variant (landmark loops of the build and the Schur complement on OpenMP
     threads; the reduced solve stays serial).  The reference's own back-end runs g2o on ONE thread, so this is extra
@@ -136,9 +148,11 @@ def run_reference(args):
     t0 = time.perf_counter()
     iters = 0
     for _ in range(args.steps):
-        _, _, st = po.optimize(pb, NUM_ITERS)
+        poses, psi, st = po.optimize(pb, NUM_ITERS)
         iters += st["iterations"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, poses, psi, st["chi2_iter"])
     v = iters / dt
     mt = cpu_mt_sample(po, pb)
     line = {
@@ -223,6 +237,8 @@ def run_ours(args):
             agg[k] += st[k]
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs and rank == 0:     # the state the last timed step left on the device, before anything else runs
+        dump_outputs(args.dump_outputs, ba.poses(), ba.points(), st["chi2_iter"])
 
     # end to end through the reference-facing call with host buffers
     e2e_iters = 0
@@ -593,7 +609,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=200, help="frames of the synthetic C3 sequence (0: skip the front-end part)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the poses, landmarks and chi2 trace of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

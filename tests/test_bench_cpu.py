@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -26,6 +28,25 @@ def test_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] == 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["cpu_baseline"]["multi_thread"]["cores"] >= 1 and d["cpu_baseline"]["multi_thread"]["value"] > 0
     assert d["e2e"] == {"value": d["value"], "unit": "iterations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_reference_arm_dumps_the_last_step(tmp_path):
+    """--dump-outputs writes what the timed step returned; the seeded C2 window makes it the oracle's result."""
+    from oracle import pyoracle as po
+    from scavislam_b200 import synth
+    r = _run(["--impl", "reference", "--steps", "1", "--warmup", "1", "--dump-outputs", str(tmp_path / "out")])
+    assert r.returncode == 0, r.stderr
+    out = {n: np.load(tmp_path / "out" / f"{n}.npy") for n in ("poses", "psi", "chi2_iter")}
+    assert all(a.dtype == np.float64 for a in out.values())
+    poses, psi, st = po.optimize(synth.make_config("C2"), 10)
+    np.testing.assert_array_equal(out["poses"], poses)
+    np.testing.assert_array_equal(out["psi"], psi)
+    np.testing.assert_array_equal(out["chi2_iter"], st["chi2_iter"])
+
+
+def test_steps_must_be_positive():
+    r = _run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr
 
 
 def test_reference_arm_other_ranks_are_silent():
