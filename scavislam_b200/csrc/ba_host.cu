@@ -113,6 +113,9 @@ struct svs_ba {
   NcclComm comm = nullptr; int comm_rank = 0, comm_size = 1;
   size_t sys_count = 0;            // doubles of the packed S | bp | bc buffer (one all-reduce per trial)
   int L_full = 0;                  // svs_ba_set_problem_sharded: landmarks of the whole window, 0 = not sharded
+  // the loaded problem is this rank's share of a sharded window: optimize() sums across the communicator only then (a
+  // whole window loaded by svs_ba_set_problem or the one-call API on a handle that has a communicator is solved alone)
+  bool sharded = false;
   double* d_psi_all = nullptr; size_t psi_all_cap = 0;
   double* d_out = nullptr; double* h_out = nullptr; size_t out_cap = 0;   // accepted state in the caller's order (one-call API)
   bool export_next = false;
@@ -208,6 +211,22 @@ int arena_reserve(svs_ba* h, size_t total, size_t upload) {
     CK(cudaMallocHost((void**)&h->stage, want));
     h->stage_cap = want;
   }
+  return SVS_OK;
+}
+
+// Observations and weights in the caller's edge order, 6 doubles per edge: pinned staging + device copy, grown on
+// demand.  A window assembled on the device (svs_ba_set_problem_from_map) never needs them, so a later host call
+// with the same structure may find them missing or too small.
+int raw_reserve(svs_ba* h, int E) {
+  const size_t need = 6 * (size_t)E;
+  if (need <= h->raw_cap) return SVS_OK;
+  if (h->d_raw) cudaFree(h->d_raw);
+  if (h->h_raw) cudaFreeHost(h->h_raw);
+  h->d_raw = h->h_raw = nullptr; h->raw_cap = 0;
+  const size_t want = need + need / 4;
+  CK(cudaMalloc((void**)&h->d_raw, want * sizeof(double)));
+  CK(cudaMallocHost((void**)&h->h_raw, want * sizeof(double)));
+  h->raw_cap = want;
   return SVS_OK;
 }
 
@@ -490,6 +509,7 @@ static int set_problem_impl(svs_ba* h, int P, const double* T_qt, const unsigned
       d.f = cam->f; d.px = cam->px; d.py = cam->py; d.b = cam->b;
       if (E > 0 && !d_obs_info) {
         // staged in pinned memory and sent in two pieces, so that the first DMA runs under the second copy
+        if (const int rc = raw_reserve(h, E)) return rc;
         const size_t bytes = 3 * (size_t)E * sizeof(double);
         const int parts = 4;
         for (int half = 0; half < 2; ++half) {
@@ -538,18 +558,8 @@ static int set_problem_impl(svs_ba* h, int P, const double* T_qt, const unsigned
   //      pinned memory and enqueues the DMA (observations, then weights) while this thread analyses the structure; a
   //      gather kernel brings them into the internal order afterwards.  The helper also keeps the copy of the index
   //      arrays that the same-structure test of the next call compares against.
-  if (E > 0 && !d_obs_info) {
-    const size_t need = 6 * (size_t)E;
-    if (need > h->raw_cap) {
-      if (h->d_raw) cudaFree(h->d_raw);
-      if (h->h_raw) cudaFreeHost(h->h_raw);
-      h->d_raw = h->h_raw = nullptr; h->raw_cap = 0;
-      const size_t want = need + need / 4;
-      CK(cudaMalloc((void**)&h->d_raw, want * sizeof(double)));
-      CK(cudaMallocHost((void**)&h->h_raw, want * sizeof(double)));
-      h->raw_cap = want;
-    }
-  }
+  if (E > 0 && !d_obs_info)
+    if (const int rc = raw_reserve(h, E)) return rc;
   struct Side {   // (every return below waits for the helper: it reads the caller's arrays)
     Worker* w;
     cudaError_t err = cudaSuccess;
@@ -870,6 +880,7 @@ static int set_problem_impl(svs_ba* h, int P, const double* T_qt, const unsigned
     sy = h->k_sy;
     h->nbranch = h->k_nbranch; h->nsep_blk = h->k_nsep;
     ++h->symbolic_hits;
+    if (host_timing) fprintf(stderr, "set_problem: symbolic factorisation reused (%d)\n", h->symbolic_hits);
   } else {
     // two concurrent branches when the window is banded and each team's share of k_solve's
     // shared-memory ring holds its widest columns, else a single chain (minimum degree order)
@@ -983,7 +994,7 @@ int svs_ba_set_problem(svs_ba* h, int P, const double* T_qt, const unsigned char
                        const double* e_info, int C, const int* c_i, const int* c_j, const double* c_T,
                        const double* c_Lambda, const svs_cam* cam) {
   svs::NvtxRange nvtx_("copyDataToG2o");
-  if (h) h->L_full = 0;
+  if (h) { h->L_full = 0; h->sharded = false; }
   return set_problem_impl(h, P, T_qt, fixed, L, psi, E, e_point, e_pose, e_anchor, e_obs, e_info, C, c_i, c_j, c_T, c_Lambda,
                           cam, nullptr);
 }
@@ -1050,8 +1061,8 @@ int svs_ba_optimize(svs_ba* h, int num_iters, int robust, double huber_delta, do
   int launches = 0;
   CKO(cudaEventRecord(h->ev[0], h->stream));
   int it = 0;
-  const NcclApi* nc = h->comm ? nccl_api() : nullptr;   // sharded window: sums across ranks on this stream
-  if (h->comm && !nc) { h->err = "NCCL library not loadable"; return -100 + SVS_ERR_STATE; }
+  const NcclApi* nc = h->comm && h->sharded ? nccl_api() : nullptr;   // sharded window: sums across ranks on this stream
+  if (h->comm && h->sharded && !nc) { h->err = "NCCL library not loadable"; return -100 + SVS_ERR_STATE; }
   const int per_trial = 2 + ((d.ntasks > 0 || d.C > 0) ? 1 : 0) + (d.ngen > 0 ? 1 : 0) + (d.nlong > 0 ? 1 : 0) + (nc ? 1 : 0);
 #define CKN(call)                                                       \
   do {                                                                  \
@@ -1427,6 +1438,7 @@ int svs_ba_set_problem_sharded(svs_ba* h, int P, const double* T_qt, const unsig
                                   li.data(), Cl, c_i, c_j, c_T, c_Lambda, cam, nullptr);
   h->extra_pairs.clear();
   h->L_full = rc == SVS_OK ? L : 0;
+  h->sharded = rc == SVS_OK;
   return rc;
 }
 
@@ -1444,8 +1456,6 @@ int svs_ba_get_points_all(svs_ba* h, double* psi) {
   if (!nc) return fail(h, SVS_ERR_STATE, "NCCL library not loadable");
   if (n > h->psi_all_cap) {
     if (h->d_psi_all) cudaFree(h->d_psi_all);
-  if (h->d_out) cudaFree(h->d_out);
-  if (h->h_out) cudaFreeHost(h->h_out);
     h->d_psi_all = nullptr; h->psi_all_cap = 0;
     CK(cudaMalloc((void**)&h->d_psi_all, n * sizeof(double)));
     h->psi_all_cap = n;
@@ -1550,6 +1560,7 @@ namespace svs {
 int ba_set_problem_device_obs(svs_ba* h, int P, const double* T_qt, const unsigned char* fixed, int L, const double* psi, int E,
                               const int* e_point, const int* e_pose, const int* e_anchor, const double* d_obs_info, int C,
                               const int* c_i, const int* c_j, const double* c_T, const double* c_Lambda, const svs_cam* cam) {
+  if (h) { h->L_full = 0; h->sharded = false; }
   const int rc = set_problem_impl(h, P, T_qt, fixed, L, psi, E, e_point, e_pose, e_anchor, nullptr, nullptr, C, c_i, c_j, c_T,
                                   c_Lambda, cam, d_obs_info);
   if (rc == SVS_OK && cudaStreamSynchronize(h->stream) != cudaSuccess) return SVS_ERR_CUDA;   // d_obs_info may be reused now

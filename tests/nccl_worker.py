@@ -1,7 +1,8 @@
 """Worker of tests/test_dist_gpu.py::test_in_library_nccl_window (launched with torch.distributed.run,
 one process per GPU): the landmark-sharded window driven INSIDE the library -- svs_ba_comm_init,
 svs_ba_set_problem_sharded, svs_ba_optimize with its per-trial ncclAllReduce -- against the CPU oracle
-on the whole window.  Prints 'NCCL_WORKER_OK' on success."""
+on the whole window.  The same handle also re-sends a window with the same structure and new numbers, and runs the
+one-call API (a whole window, no collectives) before and after the sharded loads.  Prints 'NCCL_WORKER_OK' on success."""
 import os
 import sys
 
@@ -25,11 +26,22 @@ def main():
     pb = synth.make_window(40, 3000, seed=77)
     ba = capi.BundleAdjuster(device=local)
     ba.comm_init(world, rank, ids[0])
+    rel = lambda a, b: np.abs(a - b).max() / np.abs(b).max()
+
+    def one_call(window):
+        """The one-call API on a handle that has a communicator: a whole window, solved by this rank alone."""
+        it1, T1, psi1, st1 = ba.optimise_inner_and_outer_window(window, 2)
+        T1_o, psi1_o, st1_o = po.optimize(window, 2)
+        assert it1 == st1_o["iterations"] and st1["trials_iter"] == st1_o["trials_iter"]
+        np.testing.assert_allclose(st1["chi2_iter"], st1_o["chi2_iter"], rtol=1e-7)
+        assert rel(T1, T1_o) < 1e-6 and rel(psi1, psi1_o) < 1e-6
+
+    # before the first points_all() (which sizes its own device buffer) and again at the end
+    one_call(pb)
     ba.set_problem_sharded(pb)
     it, st = ba.optimize(5)
     poses, psi = ba.poses(), ba.points_all()
     p_o, s_o, st_o = po.optimize(pb, 5)
-    rel = lambda a, b: np.abs(a - b).max() / np.abs(b).max()
     assert it == st_o["iterations"], (it, st_o["iterations"])
     assert st["trials_iter"] == st_o["trials_iter"]
     np.testing.assert_allclose(st["chi2_iter"], st_o["chi2_iter"], rtol=1e-7)
@@ -39,6 +51,18 @@ def main():
     ba.set_problem_sharded(pb)
     it2, st2 = ba.optimize(2)
     assert it2 == 2 and st2["trials_iter"] == st_o["trials_iter"][:2]
+    # the same structure with other landmarks and observations: only the numbers are sent again
+    pbn = pb.copy()
+    rng = np.random.default_rng(3)
+    pbn.psi = pb.psi * (1 + rng.normal(0, 0.02, pb.psi.shape))
+    pbn.e_obs = pb.e_obs + rng.normal(0, 0.4, pb.e_obs.shape)
+    ba.set_problem_sharded(pbn)
+    itn, stn = ba.optimize(4)
+    p_n, s_n, st_n = po.optimize(pbn, 4)
+    assert abs(st_n["chi2_final"] - st_o["chi2_iter"][3]) > 1e-5 * st_n["chi2_final"]   # stale numbers would not pass
+    assert itn == st_n["iterations"] and stn["trials_iter"] == st_n["trials_iter"]
+    np.testing.assert_allclose(stn["chi2_iter"], st_n["chi2_iter"], rtol=1e-7)
+    assert rel(ba.poses(), p_n) < 1e-6 and rel(ba.points_all(), s_n) < 1e-6
     # tracks with visibility drop-outs: every rank completes ITS tracks with zero-weight edges, so the block pattern all
     # ranks agree on must contain the pose pairs of every rank's padding (svs_ba_set_problem_sharded derives it from the
     # whole window with the same rule) -- a mismatch would sum different blocks in the all-reduce
@@ -49,6 +73,7 @@ def main():
     assert itd == st_d["iterations"] and std["trials_iter"] == st_d["trials_iter"]
     np.testing.assert_allclose(std["chi2_iter"], st_d["chi2_iter"], rtol=1e-7)
     assert rel(ba.poses(), p_d) < 1e-6 and rel(ba.points_all(), s_d) < 1e-6
+    one_call(pbn)
     ba.close()
     dist.barrier()
     dist.destroy_process_group()

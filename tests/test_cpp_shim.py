@@ -9,16 +9,22 @@ import pytest
 from scavislam_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "tests", "cpp", "shim_main")
 
 
-def _build():
-    src = os.path.join(ROOT, "tests", "cpp", "shim_main.cpp")
-    lib_dir = os.path.join(ROOT, "scavislam_b200")
-    if not os.path.exists(EXE) or os.path.getmtime(EXE) < max(os.path.getmtime(src), os.path.getmtime(os.path.join(ROOT, "include", "svs_b200.hpp"))):
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), src, "-o", EXE,
+@pytest.fixture(scope="module")
+def bin_dir(tmp_path_factory):
+    """The test programs are built outside the repository tree, which may be read-only."""
+    return tmp_path_factory.mktemp("cpp")
+
+
+def _compile(name, bin_dir):
+    src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
+    exe = str(bin_dir / name)
+    if not os.path.exists(exe):
+        lib_dir = os.path.join(ROOT, "scavislam_b200")
+        subprocess.check_call(["g++", "-std=c++17", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), src, "-o", exe,
                                "-L", lib_dir, "-lsvsb200", f"-Wl,-rpath,{lib_dir}"])
-    return EXE
+    return exe
 
 
 def _dump(pb, path):
@@ -38,9 +44,9 @@ def _dump(pb, path):
             np.ascontiguousarray(a, np.float64).tofile(f)
 
 
-def test_cpp_layer_compiles_and_fails_loudly_without_gpu(svs, tmp_path):
+def test_cpp_layer_compiles_and_fails_loudly_without_gpu(svs, tmp_path, bin_dir):
     import torch
-    exe = _build()
+    exe = _compile("shim_main", bin_dir)
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu test")
     pb = synth.make_window(4, 30, seed=2)
@@ -50,8 +56,8 @@ def test_cpp_layer_compiles_and_fails_loudly_without_gpu(svs, tmp_path):
 
 
 @pytest.mark.gpu
-def test_cpp_layer_matches_oracle(svs, oracle, tmp_path):
-    exe = _build()
+def test_cpp_layer_matches_oracle(svs, oracle, tmp_path, bin_dir):
+    exe = _compile("shim_main", bin_dir)
     pb = synth.make_config("C1")
     _dump(pb, tmp_path / "in.bin")
     r = subprocess.run([exe, str(tmp_path / "in.bin"), str(tmp_path / "out.bin"), "2"], capture_output=True, text=True)
@@ -66,30 +72,17 @@ def test_cpp_layer_matches_oracle(svs, oracle, tmp_path):
     assert np.abs(xyz - xyz_o).max() <= 1e-6 * np.abs(xyz_o).max()
 
 
-FRONTEND_EXE = os.path.join(ROOT, "tests", "cpp", "frontend_main")
-
-
-def _build_frontend():
-    src = os.path.join(ROOT, "tests", "cpp", "frontend_main.cpp")
-    lib_dir = os.path.join(ROOT, "scavislam_b200")
-    hpp = os.path.join(ROOT, "include", "svs_b200.hpp")
-    if not os.path.exists(FRONTEND_EXE) or os.path.getmtime(FRONTEND_EXE) < max(os.path.getmtime(src), os.path.getmtime(hpp)):
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), src, "-o", FRONTEND_EXE,
-                               "-L", lib_dir, "-lsvsb200", f"-Wl,-rpath,{lib_dir}"])
-    return FRONTEND_EXE
-
-
-def test_cpp_frontend_layer_compiles(svs):
-    _build_frontend()
+def test_cpp_frontend_layer_compiles(svs, bin_dir):
+    _compile("frontend_main", bin_dir)
 
 
 @pytest.mark.gpu
-def test_cpp_frontend_and_map_wrappers_equal_the_c_abi(svs, tmp_path):
+def test_cpp_frontend_and_map_wrappers_equal_the_c_abi(svs, tmp_path, bin_dir):
     """FramePreprocessor, FastGrid, DenseTracker, GuidedMatcher (corners handed over on the device),
     BA_SE3_XYZ_STEREO and DeviceMap of include/svs_b200.hpp, driven from C++ with the reference's method names, give
     what the same calls through the C ABI give (made here from Python): every wrapper is exercised, none is a shell."""
     from scavislam_b200 import frontend_inputs as fi, synth_graph, synth_images as si
-    exe = _build_frontend()
+    exe = _compile("frontend_main", bin_dir)
     seq = si.sequence(2)
     cams = fi.level_cams()
     pb = synth.make_window(12, 600, seed=9)
